@@ -4,6 +4,7 @@
     python bench.py --gpus 1 --steps 8 --warmup 3                    # our arm (CUDA path)
     python bench.py --impl reference --gpus 1 --steps 2 --warmup 1   # CPU arm: the oracle port
     torchrun --nnodes=1 --nproc-per-node N ... bench.py --gpus N ... # one rank per GPU (NCCL)
+    python bench.py --gpus 1 --steps 8 --warmup 3 --dump-outputs DIR # + the last timed step's outputs as DIR/*.npy
 
 Workload (BASELINE.json configs[1]): VQ-8192 tokenizer training, bf16 autocast, per-GPU batch 256,
 256x256 synthetic images, random-init ViT-B encoder/decoder.  One step = VQModel forward
@@ -47,7 +48,15 @@ def parse():
     p.add_argument("--no-extra", action="store_true", help="skip the MSVR10P2-4096 ours-vs-eager extra measurement")
     p.add_argument("--fp32-grads", action="store_true", help="multi-GPU: all-reduce fp32 gradient buckets (stock DDP) instead of bf16")
     p.add_argument("--cpu-sample", type=int, default=0, help="images per CPU-baseline step (0 = auto)")
-    return p.parse_args()
+    p.add_argument("--dump-outputs", type=str, default=None, metavar="DIR",
+                   help="write what the last timed step computed (losses, reconstruction, tokens, gradients, updated "
+                        "weights; fixed seeded samples of the large ones) as DIR/<name>.npy, to compare two builds")
+    a = p.parse_args()
+    if a.steps < 1 or a.warmup < 0:
+        p.error("--steps must be >= 1 and --warmup >= 0")
+    if a.dump_outputs is not None and a.impl == "reference":
+        p.error("--dump-outputs writes what a GPU arm computed: use it with --impl ours or eager")
+    return a
 
 
 # ----------------------------------------------------------------------------------------------
@@ -189,9 +198,10 @@ class Ctx:
         return [float(x) for x in t]
 
 
-def make_step(ctx, workload, B, impl):
+def make_step(ctx, workload, B, impl, keep_last=False):
     """model + optimizer + the training-step closure of one workload (the body of xqgan_train.py:448-462 restricted to
-    the in-scope path).  impl 'eager' = the reference's way of computing the path in plain PyTorch on the same GPU."""
+    the in-scope path).  impl 'eager' = the reference's way of computing the path in plain PyTorch on the same GPU.
+    keep_last: the closure keeps the forward outputs of its latest call in `step.last` (for --dump-outputs)."""
     import torch.nn.functional as F
     from imagefolder_b200 import config as xcfg
     model, margs = build_model(workload, ctx.dev)
@@ -220,6 +230,9 @@ def make_step(ctx, workload, B, impl):
         opt.zero_grad(set_to_none=True)
         loss.backward()
         opt.step()
+        if keep_last:
+            step.last = {"loss": loss, "vq_loss": vq, "commit_loss": commit, "entropy_loss": ent,
+                         "codebook_usage": usages, "reconstruction": dec}
         return loss
 
     g = torch.Generator(device=ctx.dev).manual_seed(1234 * ctx.world + ctx.rank)
@@ -260,6 +273,44 @@ def kernel_table(timing, steps):
                      "alg_bytes_per_call": nb / len(evs), "alg_flops_per_call": nf / len(evs)})
     rows.sort(key=lambda r: -r["ms_per_step"])
     return rows
+
+
+def dump_outputs(out_dir, model, last):
+    """--dump-outputs: what the last timed step handed its caller, as DIR/<name>.npy -- the losses and codebook usages
+    (float64), the reconstruction (float32), every quantizer's token indices (float64, exact), and the gradients and
+    AdamW-updated weights of all parameters in model.parameters() order (float32).  The reconstruction, gradients and
+    weights are samples at fixed seeded positions (about 33 MB in all at batch 256), the same for every run."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+
+    def save(name, t, dtype):
+        arr = t.detach().cpu().numpy() if torch.is_tensor(t) else np.asarray(t)
+        np.save(os.path.join(out_dir, name + ".npy"), arr.astype(dtype))
+
+    def sample(flat, n):
+        if flat.numel() <= n:
+            return flat
+        pos = np.sort(np.random.default_rng(0).choice(flat.numel(), n, replace=False))
+        return flat[torch.from_numpy(pos).to(flat.device)]
+
+    for k in ("loss", "vq_loss", "commit_loss", "entropy_loss"):
+        save(k, torch.as_tensor(last[k]), np.float64)
+    save("codebook_usage", [float(u) for u in last["codebook_usage"]], np.float64)
+    dec = last["reconstruction"]
+    save("reconstruction", sample(dec.float().reshape(-1), 1 << 22), np.float32)
+    tokens = []
+    for q in model._quantizers():
+        if hasattr(q, "last_idx_Bl"):
+            tokens.append(torch.cat([t.reshape(dec.shape[0], -1) for t in q.last_idx_Bl], 1))
+        elif hasattr(q, "last_idx"):
+            tokens.append(q.last_idx.reshape(dec.shape[0], -1))
+    if tokens:
+        save("tokens", torch.cat(tokens, 1), np.float64)
+    params = list(model.parameters())
+    grads = torch.cat([(p.grad if p.grad is not None else torch.zeros_like(p)).float().reshape(-1) for p in params])
+    save("grads", sample(grads, 1 << 21), np.float32)
+    del grads
+    save("params", sample(torch.cat([p.detach().float().reshape(-1) for p in params]), 1 << 21), np.float32)
 
 
 def ncu_traffic_table():
@@ -357,7 +408,7 @@ def run_ours(a):
     ctx = Ctx()
     ctx.fp32_grads = a.fp32_grads
     world, rank, local, dev = ctx.world, ctx.rank, ctx.local, ctx.dev
-    model, margs, step, imgs_dev = make_step(ctx, a.workload, a.batch, a.impl)
+    model, margs, step, imgs_dev = make_step(ctx, a.workload, a.batch, a.impl, keep_last=a.dump_outputs is not None)
     B = a.batch
     imgs_host = imgs_dev.cpu().pin_memory()
     barrier = ctx.barrier
@@ -434,6 +485,8 @@ def run_ours(a):
     e2e_steps = [round(([f0] + marks)[i].elapsed_time(marks[i]), 2) for i in range(a.steps)]
     gc.enable()
     clk = clocks.stop() if rank == 0 else None
+    if a.dump_outputs is not None and rank == 0:
+        dump_outputs(a.dump_outputs, model, step.last)
 
     ms, ms_e2e = ctx.max_over_ranks(ms, ms_e2e)
     peak_mem = torch.cuda.max_memory_allocated() / 2 ** 30

@@ -96,7 +96,7 @@ def perturbation_schedule(args, epoch: int):
 
 
 # model-relevant keys of the reference's configs/*.yaml (kept as data so tests can materialise the
-# YAMLs without the reference tree; tests/test_config.py checks them against /root/reference when present)
+# YAMLs without the reference tree; tests/test_model_cpu.py checks them against tests/golden/reference_configs.json)
 _COMMON = dict(image_size=256, vq_model="VQ-16", enc_type="dinov2", dec_type="dinov2", semantic_guide="dinov2",
                global_batch_size=1024, epochs=200, lr_scheduler="cosine", lr=3e-5, abs_pos_embed=True, ema=True,
                encoder_model="vit_base_patch14_dinov2.lvd142m", decoder_model="vit_base_patch14_dinov2.lvd142m",

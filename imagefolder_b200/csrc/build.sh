@@ -4,6 +4,8 @@ set -e
 HERE="$(cd "$(dirname "$0")" && pwd)"
 OUT="$HERE/../lib"
 mkdir -p "$OUT"
+# nvcc from PATH, else from the CUDA toolkit (a login shell does not put its bin/ on PATH)
+command -v nvcc >/dev/null || PATH="${CUDA_HOME:-/usr/local/cuda}/bin:$PATH"
 FLAGS="-gencode arch=compute_100a,code=sm_100a -O3 -lineinfo -std=c++17 -fmad=false --compiler-options -fPIC"
 nvcc $FLAGS -c "$HERE/vq_kernels.cu" -o "$OUT/vq_kernels.o" "$@" &
 nvcc $FLAGS -c "$HERE/ms_kernels.cu" -o "$OUT/ms_kernels.o" "$@" &

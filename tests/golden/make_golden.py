@@ -422,6 +422,7 @@ def main():
     case_var_helpers(VQ2, "varhelp_shared1", 8, 2, [1, 2, 4, 7], share=1, args=(128, 8), seed=12)
     case_var_helpers(LFQ, "varhelp_lfq", 10, 2, [1, 2, 3, 5], args=(2 ** 10, 10), seed=13)
     case_loss_stack()
+    case_configs()
 
 
 def case_cnn(name="cnn_small", seed=5):
@@ -442,5 +443,27 @@ def case_cnn(name="cnn_small", seed=5):
     np.savez_compressed(os.path.join(OUT, name + ".npz"), **d)
     print(name, h.shape, y.shape)
 
+
+def case_configs(name="reference_configs"):
+    """the reference's configs/*.yaml, restricted to the keys imagefolder_b200.config.SHIPPED_CONFIGS mirrors
+    (lr stays the YAML string it is there)."""
+    import glob
+    import json
+    import yaml
+    sys.path.insert(0, os.path.dirname(os.path.dirname(OUT)))
+    from imagefolder_b200.config import SHIPPED_CONFIGS
+    d = {}
+    for f in sorted(glob.glob(os.path.join(REF, "configs", "*.yaml"))):
+        cfg, y = os.path.basename(f)[:-5], yaml.safe_load(open(f))
+        d[cfg] = {k: y[k] for k in SHIPPED_CONFIGS.get(cfg, y)}
+    with open(os.path.join(OUT, name + ".json"), "w") as fh:
+        json.dump(d, fh, indent=1, sort_keys=True)
+        fh.write("\n")
+    print(name, sorted(d))
+
+
 if __name__ == "__main__":
+    if "--configs-only" in sys.argv:
+        case_configs()
+        sys.exit(0)
     main()

@@ -1,5 +1,6 @@
 """CPU tests of the host logic: config contract, VQModel wiring, and the product's ViT
 encoder/decoder against the oracle's independent restatement (same weights, fp32)."""
+import json
 import os
 
 import numpy as np
@@ -78,16 +79,16 @@ def test_yaml_contract(tmp_path):
     assert abs(al - 0.75) < 1e-12 and de == 75
 
 
-@pytest.mark.skipif(not os.path.isdir("/root/reference/configs"), reason="reference tree not present")
-def test_shipped_config_table_matches_reference_yamls():
-    import glob
-    files = sorted(glob.glob("/root/reference/configs/*.yaml"))
-    assert {os.path.basename(f)[:-5] for f in files} == set(xcfg.SHIPPED_CONFIGS)
-    for f in files:
-        y = yaml.safe_load(open(f))
-        for k, v in xcfg.SHIPPED_CONFIGS[os.path.basename(f)[:-5]].items():
+def test_shipped_config_table_matches_reference_yamls(golden_dir):
+    """golden = the reference's configs/*.yaml, one object per file holding the keys the table mirrors
+    (tests/golden/make_golden.py --configs-only)."""
+    with open(os.path.join(golden_dir, "reference_configs.json")) as f:
+        yamls = json.load(f)
+    assert set(yamls) == set(xcfg.SHIPPED_CONFIGS)
+    for name, y in yamls.items():
+        for k, v in xcfg.SHIPPED_CONFIGS[name].items():
             ref = float(y[k]) if k == "lr" else y[k]
-            assert ref == v, (f, k)
+            assert ref == v, (name, k)
 
 
 def test_model_variants_build():
