@@ -20,6 +20,7 @@
 #include "xq_tc.cuh"
 
 #include <mutex>
+#include <tuple>
 
 namespace xq {
 using namespace xqtc;
@@ -334,102 +335,11 @@ attn_fwd_kernel(const __grid_constant__ CUtensorMap tmQKV, const __grid_constant
     }
 }
 
-// The last (N mod 128) query rows when they are few (AT_TAIL_MAX): one warp per (batch*head, row) on the CUDA cores --
-// a 1-row tile would cost a full 128-row MMA tile in attn_fwd_kernel (S = 513: 20 % of its work).  Lanes split the keys,
-// each with its own online softmax, merged by shuffles at the end.  Same outputs as the tile kernel (out row, lse2).
-constexpr int AT_TAIL_MAX = 0;     // 0: ragged query tiles always run on the tile kernel (dead warps skip the softmax math)
-
-__global__ void __launch_bounds__(128)
-attn_fwd_tail_kernel(const __nv_bfloat16 *__restrict__ qkv, __nv_bfloat16 *__restrict__ out, float *__restrict__ lse2, int B, int N,
-                     int H, int n0 /* first tail row */, float c) {
-    const int lane = threadIdx.x & 31;
-    const long long w = ((long long)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
-    const int nt = N - n0;
-    if (w >= (long long)B * H * nt) return;
-    const int r = (int)(w % nt);
-    const int bh = (int)(w / nt);
-    const int b = bh / H, h = bh - b * H;
-    const int n = n0 + r;
-    const size_t W = (size_t)3 * H * AT_D;
-    const __nv_bfloat16 *qp = qkv + ((size_t)b * N + n) * W + h * AT_D;
-    float qf[AT_D];
-#pragma unroll
-    for (int u = 0; u < 8; ++u) {
-        const uint4 x = *reinterpret_cast<const uint4 *>(qp + u * 8);
-        const __nv_bfloat162 *x2 = reinterpret_cast<const __nv_bfloat162 *>(&x);
-#pragma unroll
-        for (int e = 0; e < 4; ++e) {
-            const float2 f = __bfloat1622float2(x2[e]);
-            qf[u * 8 + 2 * e] = f.x * c;             // scores directly in the log2 domain
-            qf[u * 8 + 2 * e + 1] = f.y * c;
-        }
-    }
-    float m = -CUDART_INF_F, l = 0.f, o[AT_D];
-#pragma unroll
-    for (int i = 0; i < AT_D; ++i) o[i] = 0.f;
-    for (int key = lane; key < N; key += 32) {
-        const __nv_bfloat16 *kp = qkv + ((size_t)b * N + key) * W + (H + h) * AT_D;
-        const __nv_bfloat16 *vp = kp + (size_t)H * AT_D;
-        float s = 0.f;
-#pragma unroll
-        for (int u = 0; u < 8; ++u) {
-            const uint4 x = *reinterpret_cast<const uint4 *>(kp + u * 8);
-            const __nv_bfloat162 *x2 = reinterpret_cast<const __nv_bfloat162 *>(&x);
-#pragma unroll
-            for (int e = 0; e < 4; ++e) {
-                const float2 f = __bfloat1622float2(x2[e]);
-                s = fmaf(qf[u * 8 + 2 * e], f.x, s);
-                s = fmaf(qf[u * 8 + 2 * e + 1], f.y, s);
-            }
-        }
-        const float m_new = fmaxf(m, s);
-        const float corr = ex2_approx(m - m_new);      // first key: ex2(-inf) = 0
-        const float p = ex2_approx(s - m_new);
-        l = fmaf(l, corr, p);
-        m = m_new;
-#pragma unroll
-        for (int u = 0; u < 8; ++u) {
-            const uint4 x = *reinterpret_cast<const uint4 *>(vp + u * 8);
-            const __nv_bfloat162 *x2 = reinterpret_cast<const __nv_bfloat162 *>(&x);
-#pragma unroll
-            for (int e = 0; e < 4; ++e) {
-                const float2 f = __bfloat1622float2(x2[e]);
-                o[u * 8 + 2 * e] = fmaf(o[u * 8 + 2 * e], corr, p * f.x);
-                o[u * 8 + 2 * e + 1] = fmaf(o[u * 8 + 2 * e + 1], corr, p * f.y);
-            }
-        }
-    }
-    float M = m;
-#pragma unroll
-    for (int off = 16; off > 0; off >>= 1) M = fmaxf(M, __shfl_xor_sync(0xffffffffu, M, off));
-    const float f = (m == -CUDART_INF_F) ? 0.f : ex2_approx(m - M);     // lanes without keys (N < 32) contribute nothing
-    l *= f;
-#pragma unroll
-    for (int off = 16; off > 0; off >>= 1) l += __shfl_xor_sync(0xffffffffu, l, off);
-    const float inv = 1.0f / l;
-    float mine0 = 0.f, mine1 = 0.f;
-#pragma unroll
-    for (int i = 0; i < AT_D; ++i) {
-        float x = o[i] * f;
-#pragma unroll
-        for (int off = 16; off > 0; off >>= 1) x += __shfl_xor_sync(0xffffffffu, x, off);
-        if (i == 2 * lane) mine0 = x;
-        if (i == 2 * lane + 1) mine1 = x;
-    }
-    __nv_bfloat16 *op = out + ((size_t)b * N + n) * H * AT_D + h * AT_D;
-    *reinterpret_cast<uint32_t *>(op + 2 * lane) = pack_bf16(mine0 * inv, mine1 * inv);
-    if (lane == 0) lse2[(size_t)bh * N + n] = M + log2f(l);
-}
-
 // ---- host side ------------------------------------------------------------------------------------------------------
-struct AttnMaps {
-    const void *qkv, *out;
-    int B, N, H;
-    CUtensorMap tmQKV, tmO;
-};
+struct AttnMaps { CUtensorMap tmQKV, tmO; };
 
-// per-device one-time setup (function attributes are per device; the SM count may differ between devices of one process)
-struct AttnDevState { bool fwd_attr = false, bwd_attr = false, prep_attr = false; int n_sms = 0; };
+// per-device one-time setup (function attributes are per device)
+struct AttnDevState { bool fwd_attr = false, bwd_attr = false, prep_attr = false; };
 static int attn_dev_state(AttnDevState **out) {
     static std::mutex mu;
     static AttnDevState states[64];
@@ -438,35 +348,18 @@ static int attn_dev_state(AttnDevState **out) {
     if (e != cudaSuccess) return xq::record_cuda_error(e, "cudaGetDevice");
     if (dev < 0 || dev >= 64) return XQ_ERR_UNSUPPORTED;
     std::lock_guard<std::mutex> g(mu);
-    AttnDevState &s = states[dev];
-    if (!s.n_sms) {
-        e = cudaDeviceGetAttribute(&s.n_sms, cudaDevAttrMultiProcessorCount, dev);
-        if (e != cudaSuccess) return xq::record_cuda_error(e, "cudaDeviceGetAttribute");
-    }
-    *out = &s;
+    *out = &states[dev];
     return XQ_OK;
 }
 
 static bool get_fwd_maps(const void *qkv, void *out, int B, int N, int H, AttnMaps &m) {
-    static std::mutex mu;
-    static AttnMaps cache[16];
-    static int n_cached = 0, next = 0;
-    std::lock_guard<std::mutex> g(mu);
-    for (int i = 0; i < n_cached; ++i)
-        if (cache[i].qkv == qkv && cache[i].out == out && cache[i].B == B && cache[i].N == N && cache[i].H == H) { m = cache[i]; return true; }
-    AttnMaps e;
-    e.qkv = qkv; e.out = out; e.B = B; e.N = N; e.H = H;
-    const uint64_t W = (uint64_t)3 * H * AT_D;
-    if (!make_map_3d(&e.tmQKV, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, const_cast<void *>(qkv), W, N, B, W * 2, (uint64_t)N * W * 2, AT_D, AT_BM)) return false;
-    const uint64_t Wo = (uint64_t)H * AT_D;
-    if (!make_map_3d(&e.tmO, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, out, Wo, N, B, Wo * 2, (uint64_t)N * Wo * 2, AT_D, AT_BM)) return false;
-    cache[next] = e;
-    next = (next + 1) % 16;
-    if (n_cached < 16) ++n_cached;
-    m = e;
-    return true;
+    static MapCache<std::tuple<const void *, const void *, int, int, int>, AttnMaps> cache;
+    return cache.get({qkv, out, B, N, H}, m, [&](AttnMaps &e) {
+        const uint64_t W = (uint64_t)3 * H * AT_D, Wo = (uint64_t)H * AT_D;
+        return make_map_3d(&e.tmQKV, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, const_cast<void *>(qkv), W, N, B, W * 2, (uint64_t)N * W * 2, AT_D, AT_BM) &&
+               make_map_3d(&e.tmO, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, out, Wo, N, B, Wo * 2, (uint64_t)N * Wo * 2, AT_D, AT_BM);
+    });
 }
-
 
 // =====================================================================================================================
 // Backward.  One CTA per (batch, head, 128-key block), 1 CTA per SM, looping over the query blocks i:
@@ -506,12 +399,6 @@ struct AttnBwdSmem {
     static constexpr int BAR = STAT + AB_QS * 1024;
     static constexpr int BYTES = BAR + 256;
 };
-
-__device__ __forceinline__ void bulk_load_1d(void *dst, const void *src, uint32_t bytes, uint64_t *bar) {
-    asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];"
-                 ::"r"(smem_u32(dst)), "l"(src), "r"(bytes), "r"(smem_u32(bar))
-                 : "memory");
-}
 
 // dV / dK epilogue of one item: the thread's accumulator row (64 fp32 in TMEM at `taddr`) * mul -> bf16 -> 128 contiguous bytes
 // of the packed gradient, and the column sums of the ROUNDED values of the warp's 32 rows -> qkv-bias gradient.  The sums are a
@@ -672,8 +559,8 @@ attn_bwd_kernel(const __grid_constant__ CUtensorMap tmQKV, const __grid_constant
                         mbar_expect_tx(&q_full[st], 2 * AT_TILE + 1024);
                         tma_load_3d(base + AttnBwdSmem::Q + st * AT_TILE, &tmQKV, T.colQ, i * AT_BM, T.b, &q_full[st]);
                         tma_load_3d(base + AttnBwdSmem::DO + st * AT_TILE, &tmDO, T.h * AT_D, i * AT_BM, T.b, &q_full[st]);
-                        bulk_load_1d(s_lse + st * 128, lseP + (size_t)T.bh * Npad + i * AT_BM, 512, &q_full[st]);
-                        bulk_load_1d(s_delta + st * 128, deltaP + (size_t)T.bh * Npad + i * AT_BM, 512, &q_full[st]);
+                        bulk_g2s(s_lse + st * 128, lseP + (size_t)T.bh * Npad + i * AT_BM, 512, &q_full[st]);
+                        bulk_g2s(s_delta + st * 128, deltaP + (size_t)T.bh * Npad + i * AT_BM, 512, &q_full[st]);
                     }
                     __syncwarp();
                     if (i == pre && it + (int)gridDim.x < n_items) load_kv(it + gridDim.x, n + 1);
@@ -907,10 +794,7 @@ attn_bwd_kernel(const __grid_constant__ CUtensorMap tmQKV, const __grid_constant
                     o8[g * 2 + 1] = pack_bf16(d2, d3);
                 }
                 // dS^T for the dK MMA (TMEM, over this thread's own, already consumed, dP^T columns) ...
-                asm volatile("tcgen05.st.sync.aligned.32x32b.x8.b32 [%8], {%0, %1, %2, %3, %4, %5, %6, %7};"
-                             ::"r"(o8[0]), "r"(o8[1]), "r"(o8[2]), "r"(o8[3]), "r"(o8[4]), "r"(o8[5]), "r"(o8[6]), "r"(o8[7]),
-                               "r"(tDP + lane_addr + hf * 64 + ch * 8)
-                             : "memory");
+                tmem_st8(tDP + lane_addr + hf * 64 + ch * 8, o8);
                 // ... and dS for the dQ MMA (smem, MN-major: row = key, this half's 64 queries along the row)
                 sts128(dsrow + rowtile_unit(krow, ch * 2), make_uint4(o8[0], o8[1], o8[2], o8[3]));
                 sts128(dsrow + rowtile_unit(krow, ch * 2 + 1), make_uint4(o8[4], o8[5], o8[6], o8[7]));
@@ -1227,34 +1111,19 @@ attn_dq_convert_kernel(const float *__restrict__ dq_acc, const __nv_bfloat16 *__
     }
 }
 
-struct AttnBwdMaps {
-    const void *qkv, *dout, *acc;
-    int B, N, H;
-    CUtensorMap tmQKV, tmDO, tmDQ;
-};
+struct AttnBwdMaps { CUtensorMap tmQKV, tmDO, tmDQ; };
 
 static bool get_bwd_maps(const void *qkv, const void *dout, void *acc, int B, int N, int H, AttnBwdMaps &m) {
-    static std::mutex mu;
-    static AttnBwdMaps cache[16];
-    static int n_cached = 0, next = 0;
-    std::lock_guard<std::mutex> g(mu);
-    for (int i = 0; i < n_cached; ++i)
-        if (cache[i].qkv == qkv && cache[i].dout == dout && cache[i].acc == acc && cache[i].B == B &&
-            cache[i].N == N && cache[i].H == H) { m = cache[i]; return true; }
-    AttnBwdMaps e;
-    e.qkv = qkv; e.dout = dout; e.acc = acc; e.B = B; e.N = N; e.H = H;
-    const uint64_t W = (uint64_t)3 * H * AT_D, Wo = (uint64_t)H * AT_D;
-    if (!make_map_3d(&e.tmQKV, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, const_cast<void *>(qkv), W, N, B, W * 2, (uint64_t)N * W * 2, AT_D, AT_BM)) return false;
-    if (!make_map_3d(&e.tmDO, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, const_cast<void *>(dout), Wo, N, B, Wo * 2, (uint64_t)N * Wo * 2, AT_D, AT_BM)) return false;
-    if (!make_map_3d(&e.tmDQ, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 4, acc, AT_D, N, (uint64_t)B * H, AT_D * 4, (uint64_t)N * AT_D * 4, 32, AT_BM)) return false;
-    cache[next] = e;
-    next = (next + 1) % 16;
-    if (n_cached < 16) ++n_cached;
-    m = e;
-    return true;
+    static MapCache<std::tuple<const void *, const void *, const void *, int, int, int>, AttnBwdMaps> cache;
+    return cache.get({qkv, dout, acc, B, N, H}, m, [&](AttnBwdMaps &e) {
+        const uint64_t W = (uint64_t)3 * H * AT_D, Wo = (uint64_t)H * AT_D;
+        return make_map_3d(&e.tmQKV, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, const_cast<void *>(qkv), W, N, B, W * 2, (uint64_t)N * W * 2, AT_D, AT_BM) &&
+               make_map_3d(&e.tmDO, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, const_cast<void *>(dout), Wo, N, B, Wo * 2, (uint64_t)N * Wo * 2, AT_D, AT_BM) &&
+               make_map_3d(&e.tmDQ, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, acc, AT_D, N, (uint64_t)B * H, AT_D * 4, (uint64_t)N * AT_D * 4, 32, AT_BM);
+    });
 }
 
-// keys handled by attn_bwd_ktail_kernel instead of a key block of attn_bwd_kernel (0 = none)
+// keys handled by attn_bwd_prep_kernel<NT> instead of a key block of attn_bwd_kernel (0 = none)
 static int attn_bwd_ktail(int N) {
     const int r = N % AT_BN;
     return (N > AT_BN && r != 0 && r <= AB_KTAIL_MAX) ? r : 0;
@@ -1339,7 +1208,9 @@ int xq_vit_attn_bwd(const void *qkv, const void *out, const void *d_out, const f
     }
     const long long items = (long long)B * H * nK;          // (batch*head, key block) work items of the persistent grid
     if (items > 0x7fffffffLL) return XQ_ERR_ARG;
-    const unsigned ctas = (unsigned)(items < ds->n_sms ? items : ds->n_sms);
+    int n_sm = 0;
+    XQ_CUDA_TRY(sm_count(&n_sm));
+    const unsigned ctas = (unsigned)(items < n_sm ? items : n_sm);
     attn_bwd_kernel<<<ctas, AB_THREADS, smem, st>>>(m.tmQKV, m.tmDO, m.tmDQ, lseP, deltaP, (__nv_bfloat16 *)dqkv, g_bias, N, H, nK, Npad,
                                                     (int)items, c2, scale);
     XQ_LAUNCH_CHECK("attn_bwd_kernel");
@@ -1351,13 +1222,6 @@ int xq_vit_attn_bwd(const void *qkv, const void *out, const void *d_out, const f
     return XQ_OK;
 }
 
-}  // extern "C"
-
-namespace xq {
-}  // namespace xq
-
-extern "C" {
-
 int xq_vit_attn_fwd(const void *qkv, void *out, float *lse2, int B, int N, int H, int head_dim, float scale, void *stream) {
     using namespace xq;
     if (!qkv || !out || !lse2 || B <= 0 || N <= 0 || H <= 0) return XQ_ERR_ARG;
@@ -1365,13 +1229,12 @@ int xq_vit_attn_fwd(const void *qkv, void *out, float *lse2, int B, int N, int H
     if (((uintptr_t)qkv & 15) || ((uintptr_t)out & 15)) return XQ_ERR_ARG;
     AttnMaps m;
     if (!get_fwd_maps(qkv, out, B, N, H, m)) return XQ_ERR_UNSUPPORTED;
-    // query tiles: full 128-row tiles on the tensor cores; a short remainder (<= AT_TAIL_MAX rows) on the CUDA cores
-    const int n_tail = (N % AT_BM != 0 && N % AT_BM <= AT_TAIL_MAX && N > AT_BM) ? N % AT_BM : 0;
-    const int nQ = n_tail ? N / AT_BM : (N + AT_BM - 1) / AT_BM;
+    const int nQ = (N + AT_BM - 1) / AT_BM;      // query tiles; the last one may be ragged
     const size_t smem = AttnFwdSmem::BYTES + 1024;
     AttnDevState *ds = nullptr;
     if (int rc = attn_dev_state(&ds)) return rc;
-    const int n_sm = ds->n_sms;
+    int n_sm = 0;
+    XQ_CUDA_TRY(sm_count(&n_sm));
     if (!ds->fwd_attr) {
         XQ_CUDA_TRY(cudaFuncSetAttribute(attn_fwd_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
         ds->fwd_attr = true;
@@ -1382,12 +1245,6 @@ int xq_vit_attn_fwd(const void *qkv, void *out, float *lse2, int B, int N, int H
     const float c = scale * 1.4426950408889634f;
     attn_fwd_kernel<<<grid, AT_THREADS, smem, (cudaStream_t)stream>>>(m.tmQKV, m.tmO, lse2, N, H, nQ, (int)tiles, c);
     XQ_LAUNCH_CHECK("attn_fwd_kernel");
-    if (n_tail) {
-        const long long warps = (long long)B * H * n_tail;
-        attn_fwd_tail_kernel<<<(unsigned)((warps + 3) / 4), 128, 0, (cudaStream_t)stream>>>(
-            (const __nv_bfloat16 *)qkv, (__nv_bfloat16 *)out, lse2, B, N, H, N - n_tail, c);
-        XQ_LAUNCH_CHECK("attn_fwd_tail_kernel");
-    }
     return XQ_OK;
 }
 

@@ -8,7 +8,7 @@
 // (the other four GEMMs of the block -- fc2 forward, the two weight gradients, the fc1 input gradient -- stay plain cuBLAS calls).
 //
 // C[M,N] = A[M,K] . B[N,K]^T, A and B K-major (row-major as PyTorch stores activations and Linear weights), bf16 in, fp32
-// accumulation in TMEM.  A CTA PAIR (cluster of 2) owns a 256 x 256 tile: `tcgen05.mma.cta_group::2`, M = 256 (128 accumulator
+// accumulation in TMEM.  A CTA PAIR (cluster of 2) owns a 256 x 256 tile: one `cta_group::2` MMA, M = 256 (128 accumulator
 // rows in each CTA's TMEM), N = 256 (each CTA stages half of the B tile), K = 64 per stage, 5-stage TMA ring of 32 KB per CTA,
 // accumulators double-buffered in 2 x 256 TMEM columns.  Persistent: pair p keeps column block p % (N/256) for the whole kernel
 // (bias slice in shared memory, bias-gradient sums in registers, the weight tile hot in L2) and walks the 256-row blocks.
@@ -24,6 +24,7 @@
 #include "xq_gelu.cuh"
 
 #include <mutex>
+#include <tuple>
 
 namespace xq {
 
@@ -276,53 +277,31 @@ mlp_gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__
 }
 
 // ---- host side -------------------------------------------------------------------------------------------------------
-struct GemmMaps {
-    const void *a, *b;
-    int M, N, K;
-    CUtensorMap tmA, tmB;
-};
+struct GemmMaps { CUtensorMap tmA, tmB; };
 
 static bool gm_get_maps(const void *a, const void *b, int M, int N, int K, GemmMaps &m) {
-    static std::mutex mu;
-    static GemmMaps cache[32];
-    static int n_cached = 0, next = 0;
-    std::lock_guard<std::mutex> g(mu);
-    for (int i = 0; i < n_cached; ++i)
-        if (cache[i].a == a && cache[i].b == b && cache[i].M == M && cache[i].N == N && cache[i].K == K) { m = cache[i]; return true; }
-    GemmMaps e;
-    e.a = a; e.b = b; e.M = M; e.N = N; e.K = K;
-    if (!make_map_3d(&e.tmA, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, const_cast<void *>(a), K, M, 1, (uint64_t)K * 2, (uint64_t)M * K * 2, GM_BK, GM_BM))
-        return false;
-    if (!make_map_3d(&e.tmB, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, const_cast<void *>(b), K, N, 1, (uint64_t)K * 2, (uint64_t)N * K * 2, GM_BK, GM_BN / 2))
-        return false;
-    cache[next] = e;
-    next = (next + 1) % 32;
-    if (n_cached < 32) ++n_cached;
-    m = e;
-    return true;
+    static MapCache<std::tuple<const void *, const void *, int, int, int>, GemmMaps> cache;
+    return cache.get({a, b, M, N, K}, m, [&](GemmMaps &e) {
+        return make_map_3d(&e.tmA, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, const_cast<void *>(a), K, M, 1, (uint64_t)K * 2, (uint64_t)M * K * 2, GM_BK, GM_BM) &&
+               make_map_3d(&e.tmB, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, const_cast<void *>(b), K, N, 1, (uint64_t)K * 2, (uint64_t)N * K * 2, GM_BK, GM_BN / 2);
+    });
 }
 
-struct GemmDevState { bool attr = false; int n_sms = 0; };
-static int gm_dev_state(GemmDevState **out) {
+// per-device one-time setup (function attributes are per device)
+static int gm_set_attr() {
     static std::mutex mu;
-    static GemmDevState states[64];
+    static bool attr_set[64];
     int dev = 0;
     cudaError_t e = cudaGetDevice(&dev);
     if (e != cudaSuccess) return record_cuda_error(e, "cudaGetDevice");
     if (dev < 0 || dev >= 64) return XQ_ERR_UNSUPPORTED;
     std::lock_guard<std::mutex> g(mu);
-    GemmDevState &s = states[dev];
-    if (!s.n_sms) {
-        e = cudaDeviceGetAttribute(&s.n_sms, cudaDevAttrMultiProcessorCount, dev);
-        if (e != cudaSuccess) return record_cuda_error(e, "cudaDeviceGetAttribute");
-    }
-    if (!s.attr) {
+    if (!attr_set[dev]) {
         e = cudaFuncSetAttribute(mlp_gemm_kernel<1>, cudaFuncAttributeMaxDynamicSharedMemorySize, GM_SMEM);
         if (e == cudaSuccess) e = cudaFuncSetAttribute(mlp_gemm_kernel<2>, cudaFuncAttributeMaxDynamicSharedMemorySize, GM_SMEM);
         if (e != cudaSuccess) return record_cuda_error(e, "cudaFuncSetAttribute(mlp_gemm_kernel)");
-        s.attr = true;
+        attr_set[dev] = true;
     }
-    *out = &s;
     return XQ_OK;
 }
 
@@ -336,9 +315,10 @@ static int gm_check(const void *a, const void *b, const void *c, const void *c2,
 template <int EPI>
 static int gm_launch(const void *a, const void *b, void *c, void *c2, const float *bias, float *dbias, int M, int N, int K,
                      cudaStream_t st) {
-    GemmDevState *ds = nullptr;
-    if (int rc = gm_dev_state(&ds)) return rc;
-    const int nN = N / GM_BN, max_pairs = ds->n_sms / 2;
+    if (int rc = gm_set_attr()) return rc;
+    int n_sm = 0;
+    XQ_CUDA_TRY(sm_count(&n_sm));
+    const int nN = N / GM_BN, max_pairs = n_sm / 2;
     if (nN > max_pairs) return XQ_ERR_UNSUPPORTED;
     GemmMaps m;
     if (!gm_get_maps(a, b, M, N, K, m)) return XQ_ERR_UNSUPPORTED;

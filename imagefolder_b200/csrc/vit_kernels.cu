@@ -21,8 +21,10 @@
 
 #include "../../include/xqb200.h"
 #include "xq_gelu.cuh"
+#include "xq_tc.cuh"
 
 namespace xqv {
+using namespace xqtc;
 
 constexpr int WARPS = 8;
 constexpr int THREADS = WARPS * 32;
@@ -123,31 +125,11 @@ residual_ln_fwd_kernel(const float *__restrict__ x, const __nv_bfloat16 *__restr
 
 // ---- TMA-bulk staged streaming skeleton -------------------------------------------------------------------------
 // tools/mb/stream_mb.cu (B200): a persistent 1-CTA-per-SM kernel whose producer warp stages row tiles into shared memory
-// with cp.async.bulk (1-D TMA, mbarrier complete_tx) and whose consumer warps each own one row of the tile, with tiles
+// with 1-D bulk copies (bulk_g2s, completing on an mbarrier) and whose consumer warps each own one row of the tile, with tiles
 // handed out by an atomic counter, streams at 6.7-6.8 TB/s INCLUDING register-resident column sums -- the same rate as a
 // flat copy -- where the best register-load loop (grid-stride, software-pipelined) reaches 5.7-6.0 and the previous
 // warp-per-row LayerNorm backward 4.5.  No registers are spent on loads in flight and the memory system always has
 // NST-1 tiles outstanding.
-__device__ __forceinline__ uint32_t smem_u32(const void *p) { return (uint32_t)__cvta_generic_to_shared(p); }
-__device__ __forceinline__ void mbar_init(uint64_t *bar, uint32_t count) {
-    asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(smem_u32(bar)), "r"(count));
-}
-__device__ __forceinline__ void mbar_expect_tx(uint64_t *bar, uint32_t bytes) {
-    asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(smem_u32(bar)), "r"(bytes) : "memory");
-}
-__device__ __forceinline__ void mbar_arrive(uint64_t *bar) {
-    asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(smem_u32(bar)) : "memory");
-}
-__device__ __forceinline__ void mbar_wait(uint64_t *bar, uint32_t parity) {
-    asm volatile(
-        "{\n\t.reg .pred p;\n\tXQV_WAIT:\n\t"
-        "mbarrier.try_wait.parity.shared::cta.b64 p, [%0], %1;\n\t"
-        "@p bra XQV_DONE;\n\tbra XQV_WAIT;\n\tXQV_DONE:\n\t}" ::"r"(smem_u32(bar)), "r"(parity) : "memory");
-}
-__device__ __forceinline__ void bulk_g2s(void *dst, const void *src, uint32_t bytes, uint64_t *bar) {
-    asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];"
-                 ::"r"(smem_u32(dst)), "l"(src), "r"(bytes), "r"(smem_u32(bar)) : "memory");
-}
 
 // Backward.  grid = #SMs, 1 CTA / SM, warp 0 = producer, LNB_TR consumer warps (one tile row each), LNB_NST stages.
 // Stage layout: x_out [TR][D] f32 | g_xout [TR][D] f32 | g_y [TR][D] bf16 | branch [TR][D] bf16 | mean, rstd, scale [TR].
@@ -184,7 +166,7 @@ residual_ln_bwd_kernel(const float *__restrict__ g_xout, const __nv_bfloat16 *__
     auto st_sc = [&](int st) { return reinterpret_cast<float *>(smem + st * stage_bytes + (size_t)TR * D * 12); };
     if (threadIdx.x == 0) {
         for (int i = 0; i < nst; ++i) { mbar_init(&full[i], 2); mbar_init(&empty[i], TR); }
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+        mbar_fence_init();
     }
     __syncthreads();
 
@@ -472,7 +454,7 @@ pack_qkv_kernel(const uint4 *__restrict__ dq, const uint4 *__restrict__ dk, cons
     const size_t stage_bytes = (size_t)3 * TR * src_row;           // [3][TR][C8] uint4
     if (threadIdx.x == 0) {
         for (int i = 0; i < NST; ++i) { mbar_init(&full[i], 1); mbar_init(&empty[i], TR); }
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+        mbar_fence_init();
     }
     __syncthreads();
     if (warp == 0) {
@@ -573,12 +555,11 @@ __global__ void patchify_kernel(const float *__restrict__ x, __nv_bfloat16 *__re
     store_bf16x4(out + i * 4, v);
 }
 
-// persistent grids = (SM count) x (CTAs of this kernel that are actually co-resident on one SM)
+// persistent grids = (SM count) x (CTAs of this kernel that are actually co-resident on one SM); 0 if the device query fails
 template <typename K>
 static int persistent_grid(K kernel, int threads, size_t smem = 0) {
-    int dev = 0, sms = 148, per_sm = 1;
-    cudaGetDevice(&dev);
-    cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
+    int sms = 0, per_sm = 1;
+    if (sm_count(&sms) != cudaSuccess) return 0;
     if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kernel, threads, smem) != cudaSuccess || per_sm < 1) per_sm = 1;
     return sms * per_sm;
 }
@@ -638,13 +619,6 @@ __global__ void assemble_bwd_kernel(const float *__restrict__ g, int B, int Ls, 
     if (d_table) *reinterpret_cast<float4 *>(d_table + ((size_t)t * D4 + d4) * 4) = acc;
 }
 
-static int bwd_grid() {
-    int dev = 0, sms = 148;
-    cudaGetDevice(&dev);
-    cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
-    return sms;      // 1 CTA / SM (TMA-staged tiles fill the shared memory)
-}
-
 }  // namespace xqv
 
 using namespace xqv;
@@ -659,7 +633,12 @@ using namespace xqv;
 
 extern "C" {
 
-size_t xq_vit_ln_bwd_workspace_bytes(int D) { return sizeof(float) * (size_t)bwd_grid() * NACC * D + 256; }
+// The TMA-staged kernels (LayerNorm backward, pack) run 1 CTA / SM: their tiles fill the shared memory.
+size_t xq_vit_ln_bwd_workspace_bytes(int D) {
+    int sms = 0;
+    if (sm_count(&sms) != cudaSuccess) return 0;      // xq_vit_residual_ln_bwd reports the error
+    return sizeof(float) * (size_t)sms * NACC * D + 256;
+}
 
 int xq_vit_residual_ln_fwd(const float *x, const void *branch, const float *branch_bias, const float *ls_gamma,
                            const float *rowscale, int rows_per_sample, const float *ln_w, const float *ln_b, float eps,
@@ -682,13 +661,14 @@ int xq_vit_residual_ln_bwd(const float *g_xout, const void *g_y, const float *x_
     if (!x_out || !mean || !rstd || M <= 0 || !workspace) return XQ_ERR_ARG;
     if (g_y && !ln_w) return XQ_ERR_ARG;
     if (branch && rowscale && rows_per_sample <= 0) return XQ_ERR_ARG;
-    int grid = bwd_grid();
-    if (workspace_bytes < sizeof(float) * (size_t)grid * NACC * D + 256) return XQ_ERR_WORKSPACE;
+    int sms = 0;
+    if (sm_count(&sms) != cudaSuccess) return XQ_ERR_CUDA;
+    if (workspace_bytes < sizeof(float) * (size_t)sms * NACC * D + 256) return XQ_ERR_WORKSPACE;
     const int ntiles = (M + LNB_TR - 1) / LNB_TR;
-    if (grid > ntiles) grid = ntiles;
+    const int grid = sms < ntiles ? sms : ntiles;
     cudaStream_t st = (cudaStream_t)stream;
     float *part = (float *)workspace;
-    int *counter = (int *)((char *)workspace + sizeof(float) * (size_t)bwd_grid() * NACC * D);   // dynamic tile counter
+    int *counter = (int *)((char *)workspace + sizeof(float) * (size_t)sms * NACC * D);   // dynamic tile counter
     if (cudaMemsetAsync(counter, 0, sizeof(int), st) != cudaSuccess) return XQ_ERR_CUDA;
     const int nst = lnb_stages(D);
     size_t smem = lnb_stage_bytes(D) * nst;
@@ -718,9 +698,10 @@ int xq_vit_pack_qkv(const void *dq, const void *dk, const void *dv, void *dqkv, 
     int *counter = (int *)workspace;     // dynamic tile counter, reset on the stream before each launch
     if (cudaMemsetAsync(counter, 0, sizeof(int), st) != cudaSuccess) return XQ_ERR_CUDA;
     if (g_bias && cudaMemsetAsync(g_bias, 0, sizeof(float) * 3 * (size_t)C, st) != cudaSuccess) return XQ_ERR_CUDA;
+    int sms = 0;
+    if (sm_count(&sms) != cudaSuccess) return XQ_ERR_CUDA;
     const int ntiles = (int)((M + PACK_TR - 1) / PACK_TR);
-    int grid = bwd_grid();
-    if (grid > ntiles) grid = ntiles;
+    const int grid = sms < ntiles ? sms : ntiles;
     size_t smem = (size_t)PACK_NST * 3 * PACK_TR * C8 * 16;
     const size_t red = sizeof(float) * (size_t)PACK_TR * 3 * C8 * 8;
     if (smem < red) smem = red;
@@ -778,6 +759,7 @@ int xq_vit_gelu_bwd(const void *x, const float *bias, const void *gy, void *gx, 
     int C8 = C / 8;
     int threads = C8 >= 384 ? 384 : (C8 >= 192 ? 192 : 128);
     int grid = persistent_grid(gelu_bwd_kernel, threads);
+    if (grid == 0) return XQ_ERR_CUDA;
     if ((M + GELU_BWD_RU - 1) / GELU_BWD_RU < grid) grid = (M + GELU_BWD_RU - 1) / GELU_BWD_RU;
     if (g_bias && cudaMemsetAsync(g_bias, 0, sizeof(float) * (size_t)C, st) != cudaSuccess) return XQ_ERR_CUDA;
     gelu_bwd_kernel<<<grid, threads, 0, st>>>((const uint4 *)x, bias, (const uint4 *)gy, (uint4 *)gx, g_bias, M, C8);

@@ -3,9 +3,9 @@
 // Same contract and same BIT-EXACT results as vq_search_kernel (vq_kernels.cu), reached differently:
 //
 //   screening   the -2<z,c> inner products of a 128-row x 256-code tile are computed by ONE thread issuing
-//               tcgen05.mma.kind::tf32 (operands in 128B-swizzled shared memory: rows written by the CTA,
+//               tf32 tensor-core MMAs (operands in 128B-swizzled shared memory: rows written by the CTA,
 //               code tiles streamed by TMA), accumulators in TMEM (2 x 256 columns, double buffered);
-//   epilogue    4 warps read their TMEM lanes with tcgen05.ld (32 columns at a time), take the maximum of each
+//   epilogue    4 warps read their TMEM lanes (32 columns at a time), take the maximum of each
 //               32-code group with FMNMX3 trees and remember, per row, the few groups whose maximum is
 //               within W of the running maximum (a push is ~10 instructions; no per-element scan);
 //   rescoring   only the codes of those groups (1.1 groups per row on average) are re-scored with the
@@ -18,13 +18,14 @@
 //
 // Roles (192 threads): warp 0 = TMA producer, warp 1 = TMEM allocator + MMA issuer, warps 2-5 = epilogue
 // (TMEM lane quadrant = warp_id % 4).  Pipelines: full/empty mbarriers per smem stage (TMA <-> MMA),
-// tmem_full/tmem_empty per accumulator stage (MMA <-> epilogue).
-#include <cuda.h>
-#include <mutex>
+// tmem_full/tmem_empty per accumulator stage (MMA <-> epilogue).  The PTX protocol is in xq_tc.cuh.
+#include <tuple>
 
 #include "xq_common.cuh"
+#include "xq_tc.cuh"
 
 namespace xq {
+using namespace xqtc;
 
 static long long *g_vq_tc_trace = nullptr;     // in-kernel clock trace buffer (development builds only)
 
@@ -34,90 +35,6 @@ constexpr int TC_THREADS = 192;
 constexpr int TC_CAP = 16;       // candidate-group slots per row
 constexpr float TC_EPS = 2.5e-3f;
 constexpr float TC_W = 2.0f * TC_EPS + 2e-6f;
-
-// ---- PTX wrappers ----------------------------------------------------------------------------------
-__device__ __forceinline__ uint32_t smem_u32(const void *p) { return (uint32_t)__cvta_generic_to_shared(p); }
-
-__device__ __forceinline__ void mbar_init(uint64_t *bar, uint32_t count) {
-    asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(smem_u32(bar)), "r"(count));
-}
-__device__ __forceinline__ void mbar_expect_tx(uint64_t *bar, uint32_t bytes) {
-    asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(smem_u32(bar)), "r"(bytes) : "memory");
-}
-__device__ __forceinline__ void mbar_arrive(uint64_t *bar) {
-    asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(smem_u32(bar)) : "memory");
-}
-__device__ __forceinline__ void mbar_wait(uint64_t *bar, uint32_t parity) {
-    uint32_t done;
-    do {
-        asm volatile(
-            "{\n\t.reg .pred p;\n\t"
-            "mbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2;\n\t"
-            "selp.b32 %0, 1, 0, p;\n\t}"
-            : "=r"(done)
-            : "r"(smem_u32(bar)), "r"(parity)
-            : "memory");
-    } while (!done);
-}
-__device__ __forceinline__ void tma_load_2d(void *dst, const CUtensorMap *map, int x, int y, uint64_t *bar) {
-    asm volatile(
-        "cp.async.bulk.tensor.2d.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%2, %3}], [%4];"
-        ::"r"(smem_u32(dst)), "l"(reinterpret_cast<uint64_t>(map)), "r"(x), "r"(y), "r"(smem_u32(bar))
-        : "memory");
-}
-// one lane of a CONVERGED warp: single-thread tcgen05 / TMA instructions issued under `if (lane == 0)` are wrapped by the
-// compiler in an ELECT / BRA.U.ANY serialisation loop (~112 clk per tcgen05.mma measured, tools/umma_probe.cu); issued under
-// elect.sync by a warp that runs the control flow uniformly they are plain predicated instructions (tensor-pipe rate)
-__device__ __forceinline__ bool elect_one() {
-    uint32_t pred;
-    asm volatile("{\n\t.reg .pred P;\n\telect.sync _|P, 0xffffffff;\n\tselp.b32 %0, 1, 0, P;\n\t}" : "=r"(pred));
-    return pred != 0;
-}
-__device__ __forceinline__ void tc_fence_before() { asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory"); }
-__device__ __forceinline__ void tc_fence_after() { asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory"); }
-__device__ __forceinline__ void fence_async_smem() { asm volatile("fence.proxy.async.shared::cta;" ::: "memory"); }
-
-__device__ __forceinline__ void umma_tf32(uint32_t d_tmem, uint64_t a_desc, uint64_t b_desc, uint32_t idesc, uint32_t accumulate) {
-    asm volatile(
-        "{\n\t.reg .pred p;\n\t"
-        "setp.ne.b32 p, %4, 0;\n\t"
-        "tcgen05.mma.cta_group::1.kind::tf32 [%0], %1, %2, %3, p;\n\t}"
-        ::"r"(d_tmem), "l"(a_desc), "l"(b_desc), "r"(idesc), "r"(accumulate)
-        : "memory");
-}
-__device__ __forceinline__ void umma_commit(uint64_t *bar) {
-    asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(smem_u32(bar)) : "memory");
-}
-__device__ __forceinline__ void tmem_ld32(uint32_t taddr, float (&v)[32]) {
-    uint32_t r[32];
-    asm volatile(
-        "tcgen05.ld.sync.aligned.32x32b.x32.b32 "
-        "{%0, %1, %2, %3, %4, %5, %6, %7, %8, %9, %10, %11, %12, %13, %14, %15, "
-        "%16, %17, %18, %19, %20, %21, %22, %23, %24, %25, %26, %27, %28, %29, %30, %31}, [%32];"
-        : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]), "=r"(r[4]), "=r"(r[5]), "=r"(r[6]), "=r"(r[7]), "=r"(r[8]),
-          "=r"(r[9]), "=r"(r[10]), "=r"(r[11]), "=r"(r[12]), "=r"(r[13]), "=r"(r[14]), "=r"(r[15]), "=r"(r[16]),
-          "=r"(r[17]), "=r"(r[18]), "=r"(r[19]), "=r"(r[20]), "=r"(r[21]), "=r"(r[22]), "=r"(r[23]), "=r"(r[24]),
-          "=r"(r[25]), "=r"(r[26]), "=r"(r[27]), "=r"(r[28]), "=r"(r[29]), "=r"(r[30]), "=r"(r[31])
-        : "r"(taddr));
-#pragma unroll
-    for (int i = 0; i < 32; ++i) v[i] = __uint_as_float(r[i]);
-}
-__device__ __forceinline__ void tmem_wait_ld() { asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory"); }
-
-// UMMA shared-memory descriptor: K-major operand, SWIZZLE_128B, 8-row atoms 1024 B apart.
-__device__ __forceinline__ uint64_t umma_desc_sw128(uint32_t smem_addr) {
-    uint64_t d = 0;
-    d |= (uint64_t)((smem_addr & 0x3FFFFu) >> 4);   // start address >> 4            bits [0,14)
-    d |= (uint64_t)1 << 16;                         // leading byte offset (unused for swizzled K-major)
-    d |= (uint64_t)(1024 >> 4) << 32;               // stride byte offset = 1024 B   bits [32,46)
-    d |= (uint64_t)1 << 46;                         // descriptor version (sm_100)
-    d |= (uint64_t)2 << 61;                         // layout type: SWIZZLE_128B
-    return d;
-}
-// instruction descriptor: D = F32, A = B = TF32, both K-major, M = 128, N = 256
-__host__ __device__ constexpr uint32_t umma_idesc_tf32(int M, int N) {
-    return (1u << 4) | (2u << 7) | (2u << 10) | ((uint32_t)(N >> 3) << 17) | ((uint32_t)(M >> 4) << 24);
-}
 
 // byte offset of element (row, k) inside a K-major SWIZZLE_128B operand made of 32-float (128 B) K chunks
 __device__ __forceinline__ uint32_t sw128_off(int row, int k, int rows_per_chunk) {
@@ -197,12 +114,9 @@ vq_search_tc_kernel(const __grid_constant__ CUtensorMap tmB, const float *__rest
     if (tid == 0) {
         for (int i = 0; i < nstage; ++i) { mbar_init(&s.full[i], 1); mbar_init(&s.empty[i], 1); }
         for (int i = 0; i < 2; ++i) { mbar_init(&s.tfull[i], 1); mbar_init(&s.tempty[i], 4); }
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+        mbar_fence_init();
     }
-    if (warp == 1) {
-        asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(s.tmem_ptr)), "r"(2 * TC_BN));
-        asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;");
-    }
+    if (warp == 1) tmem_alloc<2 * TC_BN>(s.tmem_ptr);
     // rows: coalesced load of the raw NCHW tile into the swizzled A operand (consecutive threads = consecutive
     // rows of one channel), then one thread per row normalises in place with the canonical chain
     for (int i = tid; i < C * TC_BM; i += TC_THREADS) {
@@ -228,7 +142,7 @@ vq_search_tc_kernel(const __grid_constant__ CUtensorMap tmB, const float *__rest
         }
         s.zz[tid] = zz;
     }
-    fence_async_smem();            // generic-proxy stores to A -> visible to the async proxy (tcgen05.mma)
+    fence_async_smem();            // generic-proxy stores to A -> visible to the async proxy (the MMAs)
     tc_fence_before();
     __syncthreads();
     tc_fence_after();
@@ -250,7 +164,7 @@ vq_search_tc_kernel(const __grid_constant__ CUtensorMap tmB, const float *__rest
         }
     } else if (warp == 1) {
         // ===== MMA issuer (whole warp runs the control flow, one elected lane issues) =====
-        const uint32_t idesc = umma_idesc_tf32(TC_BM, TC_BN);
+        const uint32_t idesc = idesc_tf32(TC_BM, TC_BN);
         const uint32_t a_addr = smem_u32(s.A);
         for (int t = 0; t < T; ++t) {
             const int st = t % nstage, as = t & 1;
@@ -265,8 +179,8 @@ vq_search_tc_kernel(const __grid_constant__ CUtensorMap tmB, const float *__rest
                 for (int kc = 0; kc < KC; ++kc) {
 #pragma unroll
                     for (int k4 = 0; k4 < 4; ++k4) {
-                        uint64_t ad = umma_desc_sw128(a_addr + kc * TC_BM * 128 + k4 * 32);
-                        uint64_t bd = umma_desc_sw128(b_addr + kc * TC_BN * 128 + k4 * 32);
+                        uint64_t ad = desc_k_sw128(a_addr + kc * TC_BM * 128 + k4 * 32);
+                        uint64_t bd = desc_k_sw128(b_addr + kc * TC_BN * 128 + k4 * 32);
                         umma_tf32(d_tmem, ad, bd, idesc, (kc | k4) ? 1u : 0u);
                     }
                 }
@@ -293,7 +207,12 @@ vq_search_tc_kernel(const __grid_constant__ CUtensorMap tmB, const float *__rest
             const int vt = t * TC_BN;
             float v[TC_BN / 32][32];
 #pragma unroll
-            for (int g = 0; g < TC_BN / 32; ++g) tmem_ld32(taddr + g * 32, v[g]);   // issue all loads, wait once
+            for (int g = 0; g < TC_BN / 32; ++g) {         // issue all loads, wait once
+                uint32_t r[32];
+                tmem_ld32(taddr + g * 32, r);
+#pragma unroll
+                for (int j = 0; j < 32; ++j) v[g][j] = __uint_as_float(r[j]);
+            }
             tmem_wait_ld();
             tc_fence_before();
             __syncwarp();
@@ -407,9 +326,7 @@ vq_search_tc_kernel(const __grid_constant__ CUtensorMap tmB, const float *__rest
     tc_fence_before();
     __syncthreads();
     tc_fence_after();
-    if (warp == 1) {
-        asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"(2 * TC_BN));
-    }
+    if (warp == 1) tmem_dealloc<2 * TC_BN>(tmem_base);
     // ---- common epilogue: z_q = normalised code (xqgan_model.py:769-771).  En[v] (prep kernel) holds exactly
     // E[v] / max(|E[v]|, eps) computed with the canonical chain, i.e. the bits the exact kernel recomputes here.
     float sq = 0.f;
@@ -471,22 +388,6 @@ __global__ void finalize_mse_tc_kernel(const float *__restrict__ partial, int n,
     }
 }
 
-typedef CUresult (*PFN_encodeTiled)(CUtensorMap *, CUtensorMapDataType, cuuint32_t, void *, const cuuint64_t *,
-                                    const cuuint64_t *, const cuuint32_t *, const cuuint32_t *, CUtensorMapInterleave,
-                                    CUtensorMapSwizzle, CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
-
-static PFN_encodeTiled get_encode_fn() {
-    static PFN_encodeTiled fn = nullptr;   // resolved once per process (a function pointer, not kernel state)
-    if (!fn) {
-        void *p = nullptr;
-        cudaDriverEntryPointQueryResult q;
-        if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &p, cudaEnableDefault, &q) == cudaSuccess &&
-            q == cudaDriverEntryPointSuccess)
-            fn = (PFN_encodeTiled)p;
-    }
-    return fn;
-}
-
 size_t vq_tc_workspace_bytes(int B, int C, int HW, int V) {
     size_t Vp = ((size_t)V + TC_BN - 1) / TC_BN * TC_BN;
     size_t ctas = ((size_t)B * HW + TC_BM - 1) / TC_BM;
@@ -503,8 +404,6 @@ int vq_tc_forward(const float *z, const float *E, int B, int C, int HW, int V, i
     if (!vq_tc_supported(C, V, 1)) return XQ_ERR_UNSUPPORTED;
     if (workspace_bytes < vq_tc_workspace_bytes(B, C, HW, V)) return XQ_ERR_WORKSPACE;
     if (((uintptr_t)workspace & 127) != 0) return XQ_ERR_UNSUPPORTED;   // TMA global address alignment
-    PFN_encodeTiled enc = get_encode_fn();
-    if (!enc) return XQ_ERR_UNSUPPORTED;
     const int Vp = (V + TC_BN - 1) / TC_BN * TC_BN;
     const int N = B * HW;
     char *ws = (char *)workspace;
@@ -518,30 +417,12 @@ int vq_tc_forward(const float *z, const float *E, int B, int C, int HW, int V, i
     if (smem > 227 * 1024) return XQ_ERR_UNSUPPORTED;
 
     // the tensor map depends only on (workspace pointer, Vp, C): encode it once per distinct triple
-    struct MapEntry { const void *ptr; int Vp, C; CUtensorMap tm; };
-    static std::mutex map_mu;
-    static MapEntry map_cache[8];
-    static int map_n = 0, map_next = 0;
+    static MapCache<std::tuple<const void *, int, int>, CUtensorMap> maps;
     CUtensorMap tm;
-    {
-        std::lock_guard<std::mutex> g(map_mu);
-        bool hit = false;
-        for (int i = 0; i < map_n && !hit; ++i)
-            if (map_cache[i].ptr == (const void *)En && map_cache[i].Vp == Vp && map_cache[i].C == C) { tm = map_cache[i].tm; hit = true; }
-        if (!hit) {
-            cuuint64_t gdim[2] = {(cuuint64_t)C, (cuuint64_t)Vp};
-            cuuint64_t gstr[1] = {(cuuint64_t)C * sizeof(float)};
-            cuuint32_t box[2] = {32u, (cuuint32_t)TC_BN};
-            cuuint32_t estr[2] = {1u, 1u};
-            CUresult r = enc(&tm, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 2, (void *)En, gdim, gstr, box, estr,
-                             CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
-                             CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-            if (r != CUDA_SUCCESS) return XQ_ERR_UNSUPPORTED;
-            map_cache[map_next] = MapEntry{(const void *)En, Vp, C, tm};
-            map_next = (map_next + 1) % 8;
-            if (map_n < 8) ++map_n;
-        }
-    }
+    if (!maps.get({En, Vp, C}, tm, [&](CUtensorMap &m) {
+            return make_map_2d(&m, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, En, C, Vp, (uint64_t)C * sizeof(float), 32, TC_BN);
+        }))
+        return XQ_ERR_UNSUPPORTED;
 
     codebook_prep_rowmajor_kernel<<<(Vp + 127) / 128, 128, 0, stream>>>(E, V, C, Vp, En, ee);
     XQ_LAUNCH_CHECK("codebook_prep_rowmajor_kernel");

@@ -290,29 +290,8 @@ gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUt
 //     peer bit cleared); the leader arms it with the pair's byte count, the peer adds a remote arrive (count 2);
 //   * only the leader issues MMAs; tcgen05.commit ... multicast::cluster arrives on the empty / tmem-full barriers of BOTH CTAs;
 //   * the epilogue warps of both CTAs hand an accumulator buffer back with a (remote) arrive on the leader's tmem-empty barrier.
+// The wrappers for these forms (cluster_ctarank, tma_load_3d_2sm, mbar_arrive_cta, umma_ss2, umma_commit2, ...) are in xq_tc.cuh.
 // =====================================================================================================================
-__device__ __forceinline__ uint32_t cluster_ctarank() { uint32_t r; asm volatile("mov.u32 %0, %%cluster_ctarank;" : "=r"(r)); return r; }
-__device__ __forceinline__ void cluster_sync_all() {
-    asm volatile("barrier.cluster.arrive.release.aligned;\n\tbarrier.cluster.wait.acquire.aligned;" ::: "memory");
-}
-__device__ __forceinline__ void tma_load_3d_2sm(void *dst, const CUtensorMap *map, int c0, int c1, int c2, uint64_t *leader_bar) {
-    asm volatile("cp.async.bulk.tensor.3d.cta_group::2.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4, %5}], [%2];"
-                 ::"r"(smem_u32(dst)), "l"(map), "r"(smem_u32(leader_bar) & 0xFEFFFFFFu), "r"(c0), "r"(c1), "r"(c2)
-                 : "memory");
-}
-__device__ __forceinline__ void mbar_arrive_cta(uint64_t *bar, uint32_t cta) {       // arrive on `bar` of cluster CTA `cta`
-    asm volatile("{\n\t.reg .b32 ra;\n\tmapa.shared::cluster.u32 ra, %0, %1;\n\tmbarrier.arrive.shared::cluster.b64 _, [ra];\n\t}"
-                 ::"r"(smem_u32(bar)), "r"(cta) : "memory");
-}
-__device__ __forceinline__ void umma_ss2(uint32_t d_tmem, uint64_t a_desc, uint64_t b_desc, uint32_t idesc, uint32_t acc) {
-    asm volatile("{\n\t.reg .pred p;\n\tsetp.ne.b32 p, %4, 0;\n\ttcgen05.mma.cta_group::2.kind::f16 [%0], %1, %2, %3, p;\n\t}"
-                 ::"r"(d_tmem), "l"(a_desc), "l"(b_desc), "r"(idesc), "r"(acc) : "memory");
-}
-__device__ __forceinline__ void umma_commit2(uint64_t *bar) {                         // arrives on `bar` in BOTH CTAs of the pair
-    asm volatile("tcgen05.commit.cta_group::2.mbarrier::arrive::one.shared::cluster.multicast::cluster.b64 [%0], %1;"
-                 ::"r"(smem_u32(bar)), "h"((uint16_t)3) : "memory");
-}
-
 #ifndef NEPI2_W
 #define NEPI2_W 16
 #endif
@@ -512,13 +491,13 @@ int main(int argc, char **argv) {
     CK(cudaMemcpy(A, hA.data(), hA.size() * 2, cudaMemcpyHostToDevice));
     CK(cudaMemcpy(B, hB.data(), hB.size() * 2, cudaMemcpyHostToDevice));
     CUtensorMap tmA, tmB;
-    if (!make_map_3d(&tmA, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, A, K, M, 1, (uint64_t)K * 2, (uint64_t)M * K * 2, BK, BM) ||
-        !make_map_3d(&tmB, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, B, K, N, 1, (uint64_t)K * 2, (uint64_t)N * K * 2, BK, BN)) {
+    if (!make_map_3d(&tmA, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, A, K, M, 1, (uint64_t)K * 2, (uint64_t)M * K * 2, BK, BM) ||
+        !make_map_3d(&tmB, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, B, K, N, 1, (uint64_t)K * 2, (uint64_t)N * K * 2, BK, BN)) {
         printf("tensor map encode failed\n");
         return 1;
     }
     CUtensorMap tmB2;
-    if (!make_map_3d(&tmB2, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, B, K, N, 1, (uint64_t)K * 2, (uint64_t)N * K * 2, BK, BN / 2)) {
+    if (!make_map_3d(&tmB2, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, B, K, N, 1, (uint64_t)K * 2, (uint64_t)N * K * 2, BK, BN / 2)) {
         printf("tensor map encode failed\n");
         return 1;
     }

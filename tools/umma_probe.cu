@@ -314,9 +314,9 @@ int main() {
         CK(cudaMemset(dout, 0, (size_t)B * N * H * 64 * 2));
         CK(cudaMemset(dacc, 0, (size_t)B * H * N * 64 * 4));
         CUtensorMap tmIn, tmOut, tmAcc;
-        bool ok = make_map_3d(&tmIn, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, dq, W, N, B, (uint64_t)W * 2, (uint64_t)N * W * 2, 64, 128);
-        ok = ok && make_map_3d(&tmOut, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, dout, H * 64, N, B, (uint64_t)H * 64 * 2, (uint64_t)N * H * 64 * 2, 64, 128);
-        ok = ok && make_map_3d(&tmAcc, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 4, dacc, 64, N, B * H, 256, (uint64_t)N * 256, 32, 128);
+        bool ok = make_map_3d(&tmIn, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, dq, W, N, B, (uint64_t)W * 2, (uint64_t)N * W * 2, 64, 128);
+        ok = ok && make_map_3d(&tmOut, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, dout, H * 64, N, B, (uint64_t)H * 64 * 2, (uint64_t)N * H * 64 * 2, 64, 128);
+        ok = ok && make_map_3d(&tmAcc, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, dacc, 64, N, B * H, 256, (uint64_t)N * 256, 32, 128);
         printf("T3 tensor maps encode: %s\n", ok ? "ok" : "FAILED");
         if (!ok) return 1;
         CK(cudaFuncSetAttribute(tma_probe_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 34816 + 1024));
