@@ -124,10 +124,11 @@ MLP_TC_ENABLED = [True]       # the tcgen05 GEMMs with fused GELU / GELU' epilog
 
 
 def mlp_tc_ok(y, fc1, fc2) -> bool:
-    """xq_vit_fc1_gelu_fwd / xq_vit_fc2_dgelu_bwd cover the shipped widths: bf16 tokens, hidden % 256 == 0, embed % 64 == 0."""
+    """xq_vit_fc1_gelu_fwd / xq_vit_fc2_dgelu_bwd cover the shipped widths: bf16 tokens, hidden % 256 == 0, in- and
+    out-features % 64 == 0 (the fc2 out-features are the K of the backward GEMM)."""
     return (MLP_TC_ENABLED[0] and y.is_cuda and y.dtype == torch.bfloat16 and fc1.bias is not None
             and fc1.weight.shape[0] % 256 == 0 and fc1.weight.shape[1] % 64 == 0 and fc1.weight.shape[0] // 256 <= 64
-            and fc2.weight.shape[1] == fc1.weight.shape[0] and fc2.weight.shape[0] % 8 == 0)
+            and fc2.weight.shape[1] == fc1.weight.shape[0] and fc2.weight.shape[0] % 64 == 0)
 
 
 class _FusedMLP(torch.autograd.Function):

@@ -170,11 +170,28 @@ def test_fused_mlp_gemm_entry_points_validate_arguments_without_gpu():
 
 
 def test_fused_mlp_dispatch_conditions():
-    """vit_ops.mlp_tc_ok: the fused GEMMs take bf16 CUDA tokens with hidden % 256 == 0 and embed % 64 == 0; everything else stays on
-    library GEMM + stand-alone bias / GELU kernel (same results, tests/test_gpu_vit_ops.py)."""
+    """vit_ops.mlp_tc_ok: the fused GEMMs take bf16 CUDA tokens with hidden % 256 == 0 and in- / out-features % 64 == 0 (the
+    out-features are the K of the fused backward GEMM, which refuses K % 64 != 0); everything else stays on library GEMM +
+    stand-alone bias / GELU kernel (same results, tests/test_gpu_vit_ops.py)."""
     import torch
     from imagefolder_b200 import vit_ops
+
+    class CudaBf16Tokens:            # the only attributes mlp_tc_ok reads from the tokens
+        is_cuda = True
+        dtype = torch.bfloat16
+
     fc1, fc2 = torch.nn.Linear(768, 3072), torch.nn.Linear(3072, 768)
     y = torch.zeros(4, 768, dtype=torch.bfloat16)
     assert not vit_ops.mlp_tc_ok(y, fc1, fc2)                          # CPU tensor: never
+    tok = CudaBf16Tokens()
+    assert vit_ops.mlp_tc_ok(tok, fc1, fc2)
+    assert vit_ops.mlp_tc_ok(tok, fc1, torch.nn.Linear(3072, 192))     # out-features != in-features, still % 64
+    for out_features in (200, 8, 96, 776):                              # % 8 == 0 but not % 64: the backward would be refused
+        assert not vit_ops.mlp_tc_ok(tok, fc1, torch.nn.Linear(3072, out_features)), out_features
+    assert not vit_ops.mlp_tc_ok(tok, torch.nn.Linear(768, 3000), torch.nn.Linear(3000, 768))   # hidden % 256 != 0
+    assert not vit_ops.mlp_tc_ok(tok, torch.nn.Linear(200, 3072), fc2)                           # in-features % 64 != 0
+    assert not vit_ops.mlp_tc_ok(tok, torch.nn.Linear(768, 3072, bias=False), fc2)               # no fc1 bias
+    f32 = CudaBf16Tokens()
+    f32.dtype = torch.float32
+    assert not vit_ops.mlp_tc_ok(f32, fc1, fc2)
     assert vit_ops.MLP_TC_ENABLED[0] is True
